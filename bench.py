@@ -25,10 +25,17 @@ sys.path.insert(0, ROOT)
 os.environ.setdefault("PYTORCH_CUDA_ALLOC_CONF", "expandable_segments:True")
 
 
+def _positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=_positive_int, default=3, help="timed GRPO steps (each of the resident and the e2e timings runs this many)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--text", default="qwen3-4b")
@@ -42,6 +49,7 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the secondary resident-row lines (16 / 32 rows per GPU)")
     ap.add_argument("--cpu-budget-s", type=float, default=25.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -133,6 +141,37 @@ def algorithmic_work(tc, dc, args):
     return dict(dense_flops=dense, decode_bytes=decode_bytes, decode_weight_bytes_per_token_step=2 * (body + head))
 
 
+DUMP_SAMPLE = 1 << 20          # at most this many of the trainable parameters / gradients are written (there are 68.7 M at config (c))
+
+
+def dump_outputs(out_dir, trainer, model, loss):
+    """What the last training step computed, as out_dir/<name>.npy (float32; the sample indices float64): its loss and metrics, the
+    rollout and scores it trained on, and a fixed seeded sample of the trainable parameters after its optimizer step and of the
+    gradients that step applied.  Two builds run with the same arguments see the same inputs, so their dumps compare entry by entry."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    step = trainer._buffered_inputs[(trainer._step - 1) % trainer.args.gradient_accumulation_steps]
+    out = {"loss": loss}
+    for k in ("kl", "clip_ratio"):
+        if trainer._metrics.get(k):
+            out[k] = trainer._metrics[k][-1]
+    for k in ("completion_ids", "completion_mask", "advantages", "ref_per_token_logps", "old_per_token_logps"):
+        if step[k] is not None:
+            out[k] = step[k]
+    ps = model.trainable_parameters()
+    params = torch.cat([p.detach().reshape(-1).float() for p in ps])
+    grads = torch.cat([p.grad.reshape(-1).float() for p in ps])
+    n = params.numel()
+    idx = torch.arange(n) if n <= DUMP_SAMPLE else torch.randint(n, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).unique()
+    out["sample_index"] = idx.double()
+    out["trainable_params_sample"] = params[idx.to(params.device)]
+    out["trainable_grads_sample"] = grads[idx.to(grads.device)]
+    for name, v in out.items():
+        a = torch.as_tensor(v).detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (a if a.dtype == torch.float64 else a.float()).numpy())
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -216,6 +255,8 @@ def run_b200(args):
         loss_host.copy_(loss.detach().reshape(1), non_blocking=False)    # D2H read of the step's result
     ms_e2e = timed(args.steps, e2e_step, tag="e2e")
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, model, loss_host)
 
     # ---- roofline of the dominant kernel: the decode weight-streaming GEMM, timed alone with CUDA events (weights of all
     #      layers = 8 GB >> 126 MB L2, so every launch reads HBM)

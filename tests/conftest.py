@@ -39,11 +39,29 @@ def golden():
 
 @pytest.fixture(scope="session")
 def tiny_oracle(golden):
-    """Oracle DNA-LLM carrying exactly the weights the reference run used."""
+    """Oracle DNA-LLM carrying exactly the weights the reference run used: regenerated from their seed, checked by digest."""
+    from bioreason_b200.configs import text_config, dna_config
+    from oracle.golden import state_sha256
+    from oracle.models import build_oracle
+    m = build_oracle(text_config("tiny"), dna_config("tiny"), seed=golden["weights_seed"])
+    assert state_sha256(m) == golden["weights_sha256"], "the seeded init no longer reproduces the reference run's weights"
+    return m.eval()
+
+
+@pytest.fixture(scope="session")
+def reference_logits(golden, tiny_oracle):
+    """Logits of the reference run (cases A and B, and A through the reference's bf16 path), recomputed by the oracle and checked
+    bit for bit against the fixture's digests."""
     import torch
     from bioreason_b200.configs import text_config, dna_config
+    from oracle.golden import tensor_sha256
     from oracle.models import build_oracle
-    m = build_oracle(text_config("tiny"), dna_config("tiny"), seed=99)   # different seed on purpose
-    missing, unexpected = m.load_state_dict({k: v.float() for k, v in golden["weights"].items()}, strict=False)
-    assert not unexpected and all("inv_freq" in k or "position_ids" in k for k in missing), (missing, unexpected)
-    return m.eval()
+    A, B = golden["A"], golden["B"]
+    # a fresh model, as the reference run built one: a used one carries its fp32 rotary cos/sin caches into bf16
+    m16 = build_oracle(text_config("tiny"), dna_config("tiny"), seed=golden["weights_seed"]).to(torch.bfloat16).eval()
+    with torch.no_grad():
+        out = {"A": tiny_oracle(**A["batch"]).logits, "B": tiny_oracle(**B["batch"]).logits, "A_bf16": m16(**A["batch"]).logits}
+    for key, want in (("A", A["logits_sha256"]), ("B", B["logits_sha256"]), ("A_bf16", A["logits_bf16_sha256"])):
+        assert tensor_sha256(out[key]) == want, f"oracle logits of case {key} differ from the reference run"
+    out["A_bf16"] = out["A_bf16"].float()
+    return out

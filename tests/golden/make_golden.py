@@ -6,8 +6,10 @@ read the fixtures.  What executes from the reference: DNALLMModel.forward / .gen
 .process_dna_embeddings (bioreason/models/dna_llm.py:103-305), DNALLMGRPOTrainer._get_per_token_logps
 and .compute_loss (grpo_trainer.py:510-520, 751-814), the EOS-mask and advantage blocks
 (grpo_trainer.py:605-609, 682-692; executed from the file's own source lines) and
-RepeatRandomSampler (:72-119).  Model weights are seeded random (no checkpoints offline) and are
-stored in the fixture (bf16-representable) so the tests do not depend on RNG reproducibility.
+RepeatRandomSampler (:72-119).  Model weights are seeded random (no checkpoints offline).  The oracle
+regenerates the weights and the logits of cases A and B exactly, so the fixture keeps the weight seed and
+SHA-256 digests of those tensors (oracle/golden.py) rather than megabytes of them; the tests recompute and
+compare the digests.
 """
 import os, sys, textwrap, types, collections
 import torch
@@ -18,6 +20,7 @@ sys.path.insert(0, ROOT); sys.path.insert(0, HERE)
 
 import _ref_import
 from bioreason_b200.configs import text_config, dna_config
+from oracle.golden import state_sha256, tensor_sha256
 from oracle.models import build_text_model, build_dna_model, round_to_bf16_, synth_batch
 
 torch.manual_seed(0)
@@ -53,9 +56,7 @@ def main():
     out = {}
     tc, dc = text_config("tiny"), dna_config("tiny")
     model = make_ref_model(tc, dc, seed=1234)
-    pnames = {n for n, _ in model.named_parameters()}
-    out["weights"] = {k: (v.to(torch.bfloat16) if k in pnames else v.clone())   # buffers (inv_freq) stay fp32
-                      for k, v in model.state_dict().items()}
+    out["weights_seed"], out["weights_sha256"] = 1234, state_sha256(model)     # oracle.models.build_oracle(..., seed=1234)
 
     # ---- case A: ragged batch, forward + CE loss (fp32 compute, bf16-representable weights)
     batch = synth_batch(tc, dc, batch=3, n_seq=2, dna_len=[12, 9, 12], text_len=[24, 17, 30], seed=11)
@@ -64,19 +65,19 @@ def main():
     labels[:, :20] = -100
     with torch.no_grad():
         o = model(**batch, labels=labels)
-    out["A"] = dict(batch=batch, labels=labels, logits=o.logits.clone(), loss=o.loss.clone())
+    out["A"] = dict(batch=batch, labels=labels, logits_sha256=tensor_sha256(o.logits), loss=o.loss.clone())
     # the reference's own --bf16 regime
     m16 = make_ref_model(tc, dc, seed=1234).to(torch.bfloat16)
     with torch.no_grad():
         o16 = m16(**batch, labels=labels)
-    out["A"]["logits_bf16"] = o16.logits.float().clone()
+    out["A"]["logits_bf16_sha256"] = tensor_sha256(o16.logits)
     out["A"]["loss_bf16"] = o16.loss.float().clone()
 
     # ---- case B: no DNA at all (dna_tokenized=None, batch_idx_map=[]) -- text-only path
     batch_b = synth_batch(tc, dc, batch=2, n_seq=0, dna_len=0, text_len=[16, 11], seed=12)
     with torch.no_grad():
         ob = model(**batch_b)
-    out["B"] = dict(batch=batch_b, logits=ob.logits.clone())
+    out["B"] = dict(batch=batch_b, logits_sha256=tensor_sha256(ob.logits))
 
     # ---- case C: count mismatch must raise ValueError (dna_llm.py:222-225)
     bad = synth_batch(tc, dc, batch=1, n_seq=1, dna_len=8, text_len=10, seed=13)

@@ -1,16 +1,15 @@
-"""SFT collate fast path (bioreason_b200/collate.py) against the reference's own loop: the label-search body of
-bioreason/dataset/kegg.py:258-323 is executed from the reference source (ast-extracted, not copied) when the tree is present, and
-against a plain restatement of it everywhere."""
-import ast
+"""SFT collate fast path (bioreason_b200/collate.py) against the reference's own loop: the labels the label-search body of
+bioreason/dataset/kegg.py:258-323 produced when executed from the reference source (recorded by tests/golden/make_source_golden.py),
+and a plain restatement of it."""
+import json
 import os
-import types
 
 import pytest
 import torch
 
 from bioreason_b200 import collate
 
-KEGG = "/root/reference/bioreason/dataset/kegg.py"
+REFERENCE = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_source.json")))
 START, END, PAD = [5, 6, 7], [9], 0
 
 
@@ -54,21 +53,13 @@ def test_labels_match_the_loop(seed):
     assert torch.equal(got, _loop_labels(ids, START, END, PAD))
 
 
-@pytest.mark.skipif(not os.path.exists(KEGG), reason="reference tree not present")
 @pytest.mark.parametrize("seed", [0, 3])
 def test_labels_match_the_reference_source(seed):
-    """Run the body of the reference's qwen_dna_collate_fn from `labels = torch.full_like(...)` to the pad mask, unmodified."""
-    tree = ast.parse(open(KEGG).read())
-    fn = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == "qwen_dna_collate_fn")
-    first = next(i for i, st in enumerate(fn.body) if isinstance(st, ast.Assign) and getattr(st.targets[0], "id", "") == "labels")
-    last = next(i for i, st in enumerate(fn.body) if isinstance(st, ast.Assign) and isinstance(st.targets[0], ast.Subscript)
-                and getattr(st.targets[0].value, "id", "") == "batch" and getattr(st.targets[0].slice, "value", "") == "labels")
-    body = fn.body[first:last]
-    ids = _random_rows(seed)
-    tok = types.SimpleNamespace(pad_token_id=PAD, encode=lambda s, add_special_tokens=False: START if "assistant" in s else END)
-    ns = {"torch": torch, "batch": {"input_ids": ids}, "processor": types.SimpleNamespace(tokenizer=tok)}
-    exec(compile(ast.Module(body=body, type_ignores=[]), KEGG, "exec"), ns)
-    assert torch.equal(collate.assistant_span_labels(ids, START, END, PAD), ns["labels"])
+    """The labels the body of the reference's qwen_dna_collate_fn, from `labels = torch.full_like(...)` to the pad mask, produced
+    unmodified on `_random_rows(seed)`."""
+    rec = REFERENCE["collate_labels"][str(seed)]
+    ids = torch.tensor(rec["input_ids"])
+    assert torch.equal(collate.assistant_span_labels(ids, START, END, PAD), torch.tensor(rec["labels"]))
 
 
 def test_placeholder_expansion_and_counts():

@@ -1,17 +1,16 @@
-"""The `peft` / `trl` stand-ins under compat/ against the reference's OWN source: `_get_target_modules` and `_prep_for_training` are
-executed from /root/reference/reason.py (extracted with ast, not copied) on a CPU stand-in that records what the kernels' LoRA
-entry point would be asked to do.  Skipped where the reference tree is absent (the GPU box)."""
-import ast
+"""The `peft` / `trl` stand-ins under compat/ against the reference's OWN source: the calls `_get_target_modules` and
+`_prep_for_training` (reason.py:362-394) make on a CPU stand-in that records what the kernels' LoRA entry point would be asked to do,
+recorded from the reference source by tests/golden/make_source_golden.py and replayed here."""
+import json
 import os
 import sys
-import types
 import weakref
 
 import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REASON = "/root/reference/reason.py"
+REFERENCE = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_source.json")))
 
 
 @pytest.fixture()
@@ -47,19 +46,22 @@ class _StandIn(torch.nn.Module):
         self.calls.append((r, alpha))
 
 
-@pytest.mark.skipif(not os.path.exists(REASON), reason="reference tree not present")
 def test_reference_prep_for_training_runs_against_the_shims(compat_path):
     import peft
-    tree = ast.parse(open(REASON).read())
-    wanted = {"_get_target_modules", "_prep_for_training"}
-    fns = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name in wanted]
-    assert {f.name for f in fns} == wanted
-    ns = {"torch": torch, "LoraConfig": peft.LoraConfig, "get_peft_model": peft.get_peft_model,
-          "prepare_model_for_kbit_training": peft.prepare_model_for_kbit_training, "DNALLMModel": _StandIn}
-    exec(compile(ast.Module(body=fns, type_ignores=[]), REASON, "exec"), ns)
-    m = _StandIn()
-    args = types.SimpleNamespace(lora_r=32, lora_alpha=64, lora_dropout=0.05)
-    cfg = ns["_prep_for_training"](m, args, dna_model_finetune=False)                             # reason.py:362-394, unmodified
+    rec = REFERENCE["prep_for_training"]
+    assert rec["training_args"] == dict(lora_r=32, lora_alpha=64, lora_dropout=0.05) and not rec["dna_model_finetune"]
+    m, objs = _StandIn(), {}
+    for op, *args in rec["calls"]:                                  # reason.py:362-394 on this stand-in, in the reference's order
+        if op == "requires_grad":
+            name, flag = args
+            for p in getattr(m, name).parameters():
+                p.requires_grad = flag
+        elif op == "LoraConfig":
+            objs[op] = peft.LoraConfig(**args[0])
+        else:                                                       # model.<module> = <peft entry point>(model.<module>, ...)
+            names = args[0]
+            setattr(m, names[0], getattr(peft, op)(*[objs[n] if n in objs else getattr(m, n) for n in names]))
+    cfg = objs[rec["returns"]]
     assert m.calls == [(32, 64.0)] and m.lora_dropout == 0.05
     assert cfg.r == 32 and {"q_proj", "k_proj", "v_proj", "o_proj", "gate_proj", "up_proj", "down_proj"} <= set(cfg.target_modules)
     assert not any(p.requires_grad for p in m.dna_model.parameters()) and all(p.requires_grad for p in m.dna_projection.parameters())

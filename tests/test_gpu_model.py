@@ -17,22 +17,22 @@ def _err_budget(test_logits, ref32, ref16, valid):
     return e_mine.max().item(), e_ref.max().item(), e_mine.mean().item(), e_ref.mean().item()
 
 
-def test_forward_tiny_golden(golden, tiny_oracle):
+def test_forward_tiny_golden(golden, tiny_oracle, reference_logits):
     from bioreason_b200.models import DNALLMModel
     m = DNALLMModel.from_oracle(tiny_oracle)
-    A = golden["A"]
+    A, ref = golden["A"], reference_logits
     out = m(**A["batch"], labels=A["labels"])
     logits = out.logits.float().cpu()
     valid = A["batch"]["attention_mask"].bool()
-    mx, rmx, mean, rmean = _err_budget(logits, A["logits"], A["logits_bf16"], valid)
-    print(f"tiny: max|err| {mx:.4g} (reference bf16 path: {rmx:.4g}); mean {mean:.4g} (ref {rmean:.4g}); logit std {A['logits'][valid].std():.3g}")
+    mx, rmx, mean, rmean = _err_budget(logits, ref["A"], ref["A_bf16"], valid)
+    print(f"tiny: max|err| {mx:.4g} (reference bf16 path: {rmx:.4g}); mean {mean:.4g} (ref {rmean:.4g}); logit std {ref['A'][valid].std():.3g}")
     assert mx <= 2.0 * rmx + 1e-3 and mean <= 2.0 * rmean + 1e-4
     assert abs(out.loss.item() - A["loss"].item()) <= 2 * abs(A["loss_bf16"].item() - A["loss"].item()) + 2e-3
     # text-only path
     Bc = golden["B"]
     lb = m(**Bc["batch"]).logits.float().cpu()
     vb = Bc["batch"]["attention_mask"].bool()
-    assert (lb - Bc["logits"])[vb].abs().max().item() <= 2.0 * rmx + 1e-3
+    assert (lb - ref["B"])[vb].abs().max().item() <= 2.0 * rmx + 1e-3
     # count mismatch raises exactly like dna_llm.py:222-225
     with pytest.raises(ValueError, match="do not match"):
         m(**golden["C"]["batch"])
